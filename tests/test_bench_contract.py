@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -15,8 +16,9 @@ def run_bench(*args):
     return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + list(args), capture_output=True, text=True, env=env, timeout=600)
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "lbm_ref_fast")), reason="oracle/_ref not built")
 def test_reference_arm_prints_one_json_line():
+    """The reference arm times the compiled reference (oracle/_ref) where it is built, the C oracle port otherwise."""
+    kind = "reference" if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "lbm_ref_fast")) else "port"
     r = run_bench("--impl", "reference", "--workload", "c1", "--steps", "4", "--warmup", "3")
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
@@ -26,7 +28,7 @@ def test_reference_arm_prints_one_json_line():
     assert j["value"] > 1.0 and j["higher_is_better"] is True and j["n_gpus"] == 1 and j["steps"] == 4 and j["warmup"] == 3
     assert j["dtype"] == "f64" and j["vs_baseline"] is None and "2048x512" in j["config"]["workload"]
     cb = j["cpu_baseline"]
-    assert cb["kind"] == "reference" and cb["cores"] >= 1 and cb["value"] == j["value"] and "2048x512" in cb["sample"]
+    assert cb["kind"] == kind and cb["cores"] >= 1 and cb["value"] == j["value"] and "2048x512" in cb["sample"]
     assert j["e2e"] == {"value": j["value"], "unit": "MLUPS", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert j["gpu_launches"] == 0
 
@@ -53,6 +55,54 @@ def test_both_arms_print_the_same_config_object():
         assert c["nx"] == 4096 * n and c["ny"] == 8192 and "exceed" in c["l2"]
     src = open(os.path.join(ROOT, "bench.py")).read()
     assert src.count('"config": config_of(cfg)') == 2  # the reference arm and the B200 arm
+
+
+def test_dump_sample_is_fixed_and_bounded():
+    """--dump-outputs samples the same cells on every run, and stays within 64 MB on the largest workload."""
+    sys.path.insert(0, ROOT)
+    import bench
+
+    a, b = bench.dump_cells(16384, 16384), bench.dump_cells(16384, 16384)
+    assert np.array_equal(a, b) and len(a) == bench.DUMP_CELLS and (np.diff(a) > 0).all() and a[-1] < 16384 * 16384
+    assert np.array_equal(bench.dump_cells(64, 32), np.arange(64 * 32))
+    assert bench.DUMP_CELLS * (3 + 2 * 9 + 2) * 8 <= 64 << 20
+
+
+DUMP_STEPS, DUMP_WARMUP = 7, 3
+
+
+@pytest.fixture(scope="module")
+def c1_oracle():
+    """The CPU oracle on c1 after the iterations bench.py runs before its dump: the untimed output period + 2, the
+    warm-up and the timed steps."""
+    from oracle import oracle as O
+
+    o = O.Oracle(O.Case(nx=2048, ny=512))
+    o.run(140 + 2 + DUMP_WARMUP + DUMP_STEPS)
+    return o
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("extra", [[], ["--aa"]], ids=["ab", "aa"])
+def test_dumped_outputs_are_the_oracles(tmp_path, c1_oracle, extra):
+    """bench.py --dump-outputs on the default cylinder flow (c1), A-B buffers and in-place AA: the sampled moments and
+    populations its timed steps leave behind are those of the CPU oracle after the same iterations."""
+    r = run_bench("--workload", "c1", "--steps", str(DUMP_STEPS), "--warmup", str(DUMP_WARMUP), "--no-cpu-baseline",
+                  "--no-e2e", "--no-parity", "--dump-outputs", str(tmp_path), *extra)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads(r.stdout)
+    assert j["steps"] == DUMP_STEPS and j["stable"]
+    got = {k: np.load(tmp_path / (k + ".npy")) for k in ("cell_x", "cell_y", "rho", "ux", "uy", "f_current", "f_next")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    x, y = got["cell_x"].astype(np.int64), got["cell_y"].astype(np.int64)
+    o = c1_oracle
+    for k in ("f_current", "f_next"):
+        ref = getattr(o, k)[y + 1, x + 1]
+        assert got[k].shape == ref.shape and (np.abs(got[k] - ref) <= 1e-12 * np.abs(ref)).all(), k
+    assert (np.abs(got["rho"] - o.rho[y, x]) <= 1e-12 * np.abs(o.rho[y, x])).all()
+    for k in ("ux", "uy"):
+        assert np.abs(got[k] - getattr(o, k)[y, x]).max() <= 1e-12, k
 
 
 @pytest.mark.parametrize("n", [1, 2, 4, 8])
