@@ -32,9 +32,10 @@ __device__ __forceinline__ void tb_kernel_body(const TbArgs& a, int p2p) {
 // Occupancy.  The skewed depth-2 march keeps two cells in registers (stage 1's loads in flight, the later stage being
 // computed): 128 registers, 512 threads = 16 warps per SM -- measured: ANY spill costs more than the warps it buys (96
 // registers / 20 warps: 42 800 MLUPS, 112 / 18: 53 300, 128 / 16: 65 800; the L1 left beside 148 KB of rings is
-// tiny).  The one-column-lag march fits 80 registers (768 threads); depth 3: 384 threads.
+// tiny).  The one-column-lag march fits 80 registers (768 threads).  Depth 3: 512 threads too, 128 registers without a
+// spill, and four blocks of 55 KB rings (lbm_tb.cuh) fit the 228 KB of an SM; the fused later stages (168 registers) 384.
 template <int T, int B, bool FORCED, bool SKEW = true, bool FUSED = false>
-__global__ void __launch_bounds__(B, (T == 3 ? 384 : ((SKEW && T == 2) || T == 1 ? TB_SKEW_THREADS : 768)) / B)
+__global__ void __launch_bounds__(B, (T == 3 ? (FUSED ? 384 : TB_SKEW_THREADS) : ((SKEW && T == 2) || T == 1 ? TB_SKEW_THREADS : 768)) / B)
     k_tb(const __grid_constant__ TbArgs a, int p2p) {
     tb_kernel_body<T, B, FORCED, SKEW, FUSED>(a, p2p);
 }
@@ -89,8 +90,7 @@ template <int T, int B, bool FORCED, bool SKEW = true, bool FUSED = false>
 cudaError_t launch_one(TbArgs a, bool p2p, cudaStream_t s) {
     using S = TbShape<T, B>;
     auto kern = k_tb<T, B, FORCED, SKEW, FUSED>;
-    // (+ 16 bytes: with fused stages the last thread of a block reads one double past its ring row, unused)
-    const size_t smem = (size_t)S::RING_DOUBLES * sizeof(double) + (FUSED ? 16 : 0);
+    const size_t smem = (size_t)S::RING_DOUBLES * sizeof(double);
     static int slots = 0;  // resident blocks on the whole device, per instantiation
     if (!slots) {
         if (smem > 48 * 1024) {
@@ -196,7 +196,7 @@ int tb_rows_per_block(int depth) {
 
 size_t tb_shared_bytes(int depth) {
     const int b = block_threads();
-    return (size_t)(depth - 1) * TB_SLOTS * Q * b * sizeof(double);
+    return (size_t)(depth - 1) * TB_RING_PLANES * b * sizeof(double);
 }
 
 cudaError_t launch_macros_finish(const ObserveArgs& o, const double* m_rho, const double* m_ux, const double* m_uy,

@@ -8,7 +8,8 @@
 //   stage k   updates column s-2(k-1)     from stage k-1's ring in SHARED MEMORY (iteration t+k-1)
 //   stage T   stores column s-2(T-1)      to the destination buffer in HBM
 // so each population is read once and written once per T updates: 144/T B per update.  A stage's ring
-// holds its last four columns (a pull needs the three columns c-1, c, c+1).  Because stage k lags TWO
+// holds each population of a column until the next stage has pulled it (a pull needs the three columns c-1, c, c+1):
+// two, three or four columns, depending on the population (see "the ring" below).  Because stage k lags TWO
 // columns behind stage k-1, everything it reads was written in earlier steps: the stages of a step are
 // independent, stage 1's loads fly while the later stages compute, and one __syncthreads ends the step.
 // (The one-column-lag march -- stage k on column s-(k-1), a barrier between the stages, stage 1's loads
@@ -50,8 +51,81 @@ enum TbEdge {
     TB_EDGE_WRAP = 2    // periodic in x inside one slab: column indices wrap
 };
 
-constexpr int TB_SLOTS = 4;       // ring slots per stage
 constexpr int TB_MAX_DEPTH = 3;   // == Layout::XO + 1 ghost columns are addressable
+
+// ---- the ring ------------------------------------------------------------------------------------
+// Stage k < T keeps the columns it computed in a ring in shared memory until stage k+1 has pulled them.  How long
+// depends on the population.  In the skewed march stage k+1 pulls populations 3, 6, 7 (from x+1) of a column one
+// step after it was stored, 0, 2, 4 (from x) two steps after and 1, 5, 8 (from x-1) three steps after; a column
+// stored in step s is therefore dead after step s+1, s+2, s+3, and since a step has no barrier inside, it must not
+// share a slot with the column stored in that last step either.  So the ring is three GROUPS, g = 0 (3, 6, 7),
+// 1 (0, 2, 4), 2 (1, 5, 8), with g + 2 slots each, and the column stored in step s goes to slot s mod (g + 2) of
+// every group: 27 planes of B doubles per stage instead of 4 x 9 (four depth-3 blocks of 128 rows fit an SM).  The
+// one-column-lag march pulls one step earlier, after a barrier, and fits the same slots (tb_slots; both marches are
+// replayed by tests/cpp/tb_ring_schedule.cpp).
+// A slot is three planes of B doubles (one row per thread), in the order (row offset of the pull) +1, 0, -1:
+//   group 0: 7, 3, 6   group 1: 4, 0, 2   group 2: 8, 1, 5
+// so that the +-1-row reads of the first and last thread of a block (dead rows, computed by the fused lane) stay
+// inside the slot and the ring needs no guard at its end.
+constexpr int TB_RING_PLANES = 27;  // per stage
+
+LBM_HD constexpr int tb_ring_slots(int g) { return g + 2; }
+
+// Offset in doubles of the slot of group g in stage k's ring (1 <= k < T) that holds the column stored in march
+// step s, row 0 (add the thread's row).
+template <int B>
+LBM_HD constexpr int tb_ring_at(int k, int g, int s) {
+    const int n = tb_ring_slots(g);
+    int slot = s % n;
+    if (slot < 0) slot += n;
+    return ((k - 1) * TB_RING_PLANES + 3 * (g * (g + 3) / 2 + slot)) * B;
+}
+
+// The slot term of tb_ring_at: offset of the slot that holds the column stored in step s from slot 0 of its group.
+template <int B>
+LBM_HD int tb_ring_slot(int g, int s) {
+    return tb_ring_at<B>(1, g, s) - tb_ring_at<B>(1, g, 0);
+}
+
+// Stage k+1's pull of one cell (column c) out of stage k's ring / stage k's store of one cell into it.  o0, o1, o2:
+// the slot offsets (tb_ring_slot) of group 0 / 1 / 2, i.e. of columns c+1, c, c-1 for the pull; rt = ring + tid.
+template <int B>
+LBM_HD void tb_ring_pull(const double* rt, int k, int o0, int o1, int o2, double f[Q]) {
+    const double* e = rt + tb_ring_at<B>(k, 0, 0) + o0;
+    const double* z = rt + tb_ring_at<B>(k, 1, 0) + o1;
+    const double* w = rt + tb_ring_at<B>(k, 2, 0) + o2;
+    f[7] = e[1];
+    f[3] = e[B];
+    f[6] = e[2 * B - 1];
+    f[4] = z[1];
+    f[0] = z[B];
+    f[2] = z[2 * B - 1];
+    f[8] = w[1];
+    f[1] = w[B];
+    f[5] = w[2 * B - 1];
+}
+template <int B>
+LBM_HD void tb_ring_put(double* rt, int k, int o0, int o1, int o2, const double f[Q]) {
+    double* e = rt + tb_ring_at<B>(k, 0, 0) + o0;
+    double* z = rt + tb_ring_at<B>(k, 1, 0) + o1;
+    double* w = rt + tb_ring_at<B>(k, 2, 0) + o2;
+    e[0] = f[7];
+    e[B] = f[3];
+    e[2 * B] = f[6];
+    z[0] = f[4];
+    z[B] = f[0];
+    z[2 * B] = f[2];
+    w[0] = f[8];
+    w[B] = f[1];
+    w[2 * B] = f[5];
+}
+
+// One cell's populations into every slot of stage k's ring (steps 0 .. 3 cover the slots of every group).
+template <int B>
+LBM_HD void tb_ring_fill(double* rt, int k, const double f[Q]) {
+#pragma unroll 1
+    for (int s = 0; s < tb_ring_slots(2); ++s) tb_ring_put<B>(rt, k, tb_ring_slot<B>(0, s), tb_ring_slot<B>(1, s), tb_ring_slot<B>(2, s), f);
+}
 
 struct TbArgs {
     const double* src;
@@ -147,7 +221,7 @@ template <int T, int B>
 struct TbShape {
     static constexpr int ROFF = (T == 1) ? 0 : 2;  // thread j works on row strip*H - ROFF + j
     static constexpr int H = B - 2 * ROFF;         // rows a strip stores (a multiple of four: whole 32-byte sectors)
-    static constexpr int RING_DOUBLES = (T - 1) * TB_SLOTS * Q * B;
+    static constexpr int RING_DOUBLES = tb_ring_at<B>(T, 0, 0);  // the rings of stages 1 .. T-1
     static_assert(T >= 1 && T <= TB_MAX_DEPTH, "depth");
     static_assert(ROFF >= T - 1, "row overlap");
 };
@@ -251,39 +325,50 @@ LBM_HD void tb_issue(const TbArgs& a, const TbRow<T, B>& r, int c, bool masked, 
     }
 }
 
-// Stage k >= 2, first half: the same cell from stage k-1's ring in shared memory.
-template <int T, int B, bool PLAIN>
-LBM_HD void tb_from_ring(const TbArgs& a, const TbRow<T, B>& r, const double* ring, int k, int c, bool masked, TbCell& cell) {
-    tb_classify<T, B, PLAIN>(a, r, k, c, masked, cell);
-    if (cell.kind != 1) return;
-    const double* g = ring + (k - 2) * (TB_SLOTS * Q * B) + r.tid;
-    const double* gw = g + ((c - 1) & (TB_SLOTS - 1)) * (Q * B);
-    const double* g0 = g + (c & (TB_SLOTS - 1)) * (Q * B);
-    const double* ge = g + ((c + 1) & (TB_SLOTS - 1)) * (Q * B);
-    cell.f[0] = g0[0 * B];
-    cell.f[1] = gw[1 * B];
-    cell.f[2] = g0[2 * B - 1];
-    cell.f[3] = ge[3 * B];
-    cell.f[4] = g0[4 * B + 1];
-    cell.f[5] = gw[5 * B - 1];
-    cell.f[6] = ge[6 * B - 1];
-    cell.f[7] = ge[7 * B + 1];
-    cell.f[8] = gw[8 * B + 1];
+// The ring slots a march step uses (uniform): every stage stores into st[g] (tb_ring_slot of the step) and pulls from
+// pl[g].  The skewed march pulls from group g the column stored g + 1 steps before, the one-column-lag march
+// (a barrier between the stages) the one stored g steps before: slot s+1 resp. s+2 mod (g + 2).
+struct TbSlots {
+    int st[3], pl[3];
+};
+template <int B>
+LBM_HD TbSlots tb_slots(int s, bool skew) {
+    TbSlots o;
+#pragma unroll
+    for (int g = 0; g < 3; ++g) {
+        o.st[g] = tb_ring_slot<B>(g, s);
+        o.pl[g] = tb_ring_slot<B>(g, s + (skew ? 1 : 2));
+    }
+    return o;
+}
+// ... of the next step of the skewed march: the slots pulled from become the ones stored into
+template <int B>
+LBM_HD void tb_slots_advance(TbSlots& o) {
+#pragma unroll
+    for (int g = 0; g < 3; ++g) {
+        o.st[g] = o.pl[g];
+        o.pl[g] = o.pl[g] + 3 * B == tb_ring_slots(g) * 3 * B ? 0 : o.pl[g] + 3 * B;
+    }
 }
 
-// (cold, kept out of line: the hot loop should fit the instruction cache) a constant cell into stage k's ring
-// which: 2 eq(1,u_in,0), 3 zero, 4 w (the kinds of TbCell).  `a` is a __grid_constant__ kernel parameter: taking its
-// address costs nothing.
+// Stage k >= 2, first half: the same cell from stage k-1's ring in shared memory.
+template <int T, int B, bool PLAIN>
+LBM_HD void tb_from_ring(const TbArgs& a, const TbRow<T, B>& r, const double* ring, int k, int c, const TbSlots& o,
+                         bool masked, TbCell& cell) {
+    tb_classify<T, B, PLAIN>(a, r, k, c, masked, cell);
+    if (cell.kind != 1) return;
+    tb_ring_pull<B>(ring + r.tid, k - 1, o.pl[0], o.pl[1], o.pl[2], cell.f);
+}
+
+// (cold, kept out of line: the hot loop should fit the instruction cache) a constant cell into stage k's ring, slots
+// o0, o1, o2.  which: 2 eq(1,u_in,0), 3 zero, 4 w (the kinds of TbCell).  `a` is a __grid_constant__ kernel parameter:
+// taking its address costs nothing.
 template <int B>
-TB_COLD void tb_ring_const(double* w, const TbArgs& a, int which) {
-    if (which == 3) {
+TB_COLD void tb_ring_const(double* rt, int k, int o0, int o1, int o2, const TbArgs& a, int which) {
+    double v[Q];
 #pragma unroll
-        for (int i = 0; i < Q; ++i) w[i * B] = 0.0;
-        return;
-    }
-    const double* v = which == 2 ? a.bc.e : a.bc.w;
-#pragma unroll
-    for (int i = 0; i < Q; ++i) w[i * B] = v[i];
+    for (int i = 0; i < Q; ++i) v[i] = which == 3 ? 0.0 : (which == 2 ? a.bc.e[i] : a.bc.w[i]);
+    tb_ring_put<B>(rt, k, o0, o1, o2, v);
 }
 
 // The last stage's populations of an edge column into the neighbours' ghost columns (peer memory over NVLink).
@@ -330,19 +415,18 @@ LBM_HD void tb_push(const TbArgs& a, const TbRow<T, B>& r, int c, const double* 
     }
 }
 
-// Second half of every stage: boundary rules, stability check, collision; then the ring (k < T) or HBM and the
-// neighbours' ghost columns (k == T).  Returns true when a checked value was unstable.
+// Second half of every stage: boundary rules, stability check, collision; then the ring (k < T, slots o.st) or HBM and
+// the neighbours' ghost columns (k == T).  Returns true when a checked value was unstable.
 template <int T, int B, bool FORCED, bool PLAIN>
-LBM_HD bool tb_finish(const TbArgs& a, const TbRow<T, B>& r, double* ring, int k, int c, TbCell& cell) {
+LBM_HD bool tb_finish(const TbArgs& a, const TbRow<T, B>& r, double* ring, int k, int c, const TbSlots& o, TbCell& cell) {
     const Layout& L = a.L;
     const int lnx = L.lnx, ny = L.ny;
     if (cell.kind == 0) return false;
-    double* w = ring + (k - 1) * (TB_SLOTS * Q * B) + (c & (TB_SLOTS - 1)) * (Q * B) + r.tid;  // (k < T only)
     if (cell.kind != 1) {
         // ---- cold: constants.  Written from the argument block straight to the ring: nothing is merged into the
         // registers of the hot path.
         if (k < T) {
-            tb_ring_const<B>(w, a, cell.kind);
+            tb_ring_const<B>(ring + r.tid, k, o.st[0], o.st[1], o.st[2], a, cell.kind);
         } else if (cell.kind == 4) {
             if (a.m_rho) {  // include/LBMSolver.h:260-261; rho keeps the constructor's 1.0
                 const long long g = (long long)c * ny + r.y;
@@ -381,7 +465,7 @@ LBM_HD bool tb_finish(const TbArgs& a, const TbRow<T, B>& r, double* ring, int k
         // ---- cold: an obstacle cell with a fluid neighbour: checked (the reference's check sees what streams into
         // it), then w for ever (SURVEY.md F3)
         if (k < T) {
-            tb_ring_const<B>(w, a, 4);
+            tb_ring_const<B>(ring + r.tid, k, o.st[0], o.st[1], o.st[2], a, 4);
         } else {
             if (a.m_rho) {
                 const long long g = (long long)c * ny + r.y;
@@ -413,8 +497,7 @@ LBM_HD bool tb_finish(const TbArgs& a, const TbRow<T, B>& r, double* ring, int k
         else
             bgk(f, mo, a.tau_inv, f);
         if (k < T) {
-#pragma unroll
-            for (int i = 0; i < Q; ++i) w[i * B] = f[i];
+            tb_ring_put<B>(ring + r.tid, k, o.st[0], o.st[1], o.st[2], f);
             return bad;
         }
         if (!a.write) return bad;
@@ -452,12 +535,13 @@ LBM_HD void tb_step(const TbArgs& a, const TbRow<T, B>& r, double* ring, int s, 
                     TbCell& nxt, bool bad[T]) {
     if (r.tid == 0 && r.pf_bytes > 0 && s + 1 + a.pf_dist <= r.pf_last) tb_prefetch_l2<T, B>(a, r.pf_seg, r.pf_bytes, s + 1 + a.pf_dist);
     if (issue_next) tb_issue<T, B, PLAIN>(a, r, s + 1, masked, nxt);
-    bad[0] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, 1, s, cur);
+    const TbSlots o = tb_slots<B>(s, false);
+    bad[0] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, 1, s, o, cur);
 #pragma unroll
     for (int k = 2; k <= T; ++k) {
         TB_SYNC();  // stage k-1's column of this step is in its ring
-        tb_from_ring<T, B, PLAIN>(a, r, ring, k, s - (k - 1), masked, cur);
-        bad[k - 1] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, k, s - (k - 1), cur);
+        tb_from_ring<T, B, PLAIN>(a, r, ring, k, s - (k - 1), o, masked, cur);
+        bad[k - 1] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, k, s - (k - 1), o, cur);
     }
 }
 
@@ -471,13 +555,14 @@ LBM_HD void tb_step_skew(const TbArgs& a, const TbRow<T, B>& r, double* ring, in
     if (r.tid == 0 && r.pf_bytes > 0 && s + a.pf_dist <= r.pf_last) tb_prefetch_l2<T, B>(a, r.pf_seg, r.pf_bytes, s + a.pf_dist);
     TbCell first;
     tb_issue<T, B, PLAIN>(a, r, s, masked, first);
+    const TbSlots o = tb_slots<B>(s, true);
 #pragma unroll
     for (int k = T; k >= 2; --k) {
         TbCell cell;
-        tb_from_ring<T, B, PLAIN>(a, r, ring, k, s - 2 * (k - 1), masked, cell);
-        bad[k - 1] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, k, s - 2 * (k - 1), cell);
+        tb_from_ring<T, B, PLAIN>(a, r, ring, k, s - 2 * (k - 1), o, masked, cell);
+        bad[k - 1] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, k, s - 2 * (k - 1), o, cell);
     }
-    bad[0] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, 1, s, first);
+    bad[0] |= tb_finish<T, B, FORCED, PLAIN>(a, r, ring, 1, s, o, first);
     if (T > 1) TB_SYNC();
 }
 
@@ -566,6 +651,7 @@ LBM_HD void tb_fast_lane(const TbArgs& a, const TbRow<T, B>& r, double* ring, in
     const char* pl = tb_opaque(r.srow + (long long)(s + 1 + Layout::XO) * a.col_bytes);
     char* ps = tb_opaque(r.drow + (long long)(s - 2 * (T - 1) + 1 + Layout::XO) * a.col_bytes);
     double* const rt = ring + r.tid;
+    TbSlots o = tb_slots<B>(s, true);  // (uniform, advanced by one slot per step)
     for (; s < s_end; ++s) {
         if (pfp && s + a.pf_dist <= r.pf_last) TB_PREFETCH_L2(pfp);
         // stage k works on column s - 2(k-1) while that lies in its range [x0 - (T-k), x1 + (T-k)) (uniform)
@@ -581,26 +667,12 @@ LBM_HD void tb_fast_lane(const TbArgs& a, const TbRow<T, B>& r, double* ring, in
         for (int k = T; k >= 2; --k) {
             if (!now[k - 1]) continue;
             const int c = s - 2 * (k - 1);
-            const double* g = rt + (k - 2) * (TB_SLOTS * Q * B);
-            const double* gw = g + ((c - 1) & (TB_SLOTS - 1)) * (Q * B);
-            const double* g0 = g + (c & (TB_SLOTS - 1)) * (Q * B);
-            const double* ge = g + ((c + 1) & (TB_SLOTS - 1)) * (Q * B);
             double f[Q];
-            f[0] = g0[0 * B];
-            f[1] = gw[1 * B];
-            f[2] = g0[2 * B - 1];
-            f[3] = ge[3 * B];
-            f[4] = g0[4 * B + 1];
-            f[5] = gw[5 * B - 1];
-            f[6] = ge[6 * B - 1];
-            f[7] = ge[7 * B + 1];
-            f[8] = gw[8 * B + 1];
+            tb_ring_pull<B>(rt, k - 1, o.pl[0], o.pl[1], o.pl[2], f);
             Moments mo;
             bad[k - 1] |= tb_fast_cell<FORCED>(a, r.strip_walls, r.wall_b, r.wall_t, f, mo);
             if (k < T) {
-                double* w = rt + (k - 1) * (TB_SLOTS * Q * B) + (c & (TB_SLOTS - 1)) * (Q * B);
-#pragma unroll
-                for (int i = 0; i < Q; ++i) w[i * B] = f[i];
+                tb_ring_put<B>(rt, k, o.st[0], o.st[1], o.st[2], f);
             } else {
                 if (a.m_rho) {  // (uniform; the last pass before an output only)
                     const long long g = (long long)c * a.L.ny + r.y;
@@ -615,9 +687,7 @@ LBM_HD void tb_fast_lane(const TbArgs& a, const TbRow<T, B>& r, double* ring, in
             Moments mo;
             bad[0] |= tb_fast_cell<FORCED>(a, r.strip_walls, r.wall_b, r.wall_t, f1, mo);
             if (T > 1) {
-                double* w = rt + (s & (TB_SLOTS - 1)) * (Q * B);
-#pragma unroll
-                for (int i = 0; i < Q; ++i) w[i * B] = f1[i];
+                tb_ring_put<B>(rt, 1, o.st[0], o.st[1], o.st[2], f1);
             } else {
                 if (a.m_rho) {
                     const long long g = (long long)s * a.L.ny + r.y;
@@ -631,6 +701,7 @@ LBM_HD void tb_fast_lane(const TbArgs& a, const TbRow<T, B>& r, double* ring, in
         pl = tb_opaque(pl + a.col_bytes);
         ps = tb_opaque(ps + a.col_bytes);
         if (pfp) pfp = tb_opaque(pfp + a.col_bytes);
+        tb_slots_advance<B>(o);
         if (T > 1) TB_SYNC();
     }
 }
@@ -660,6 +731,7 @@ LBM_HD void tb_fast_lane_fused(const TbArgs& a, const TbRow<T, B>& r, double* ri
     const char* pl = tb_opaque(r.srow + (long long)(s + 1 + Layout::XO) * a.col_bytes);
     char* ps = tb_opaque(r.drow + (long long)(s - 2 * (T - 1) + 1 + Layout::XO) * a.col_bytes);
     double* const rt = ring + r.tid;
+    TbSlots o = tb_slots<B>(s, true);
     for (; s < s_end; ++s) {
         if (pfp && s + a.pf_dist <= r.pf_last) TB_PREFETCH_L2(pfp);
         double f1[Q];
@@ -669,22 +741,7 @@ LBM_HD void tb_fast_lane_fused(const TbArgs& a, const TbRow<T, B>& r, double* ri
         Moments mo[K];
         bool window = true;
 #pragma unroll
-        for (int j = K - 1; j >= 0; --j) {
-            const int c = s - 2 * (j + 1);
-            const double* g = rt + j * (TB_SLOTS * Q * B);
-            const double* gw = g + ((c - 1) & (TB_SLOTS - 1)) * (Q * B);
-            const double* g0 = g + (c & (TB_SLOTS - 1)) * (Q * B);
-            const double* ge = g + ((c + 1) & (TB_SLOTS - 1)) * (Q * B);
-            f[j][0] = g0[0 * B];
-            f[j][1] = gw[1 * B];
-            f[j][2] = g0[2 * B - 1];
-            f[j][3] = ge[3 * B];
-            f[j][4] = g0[4 * B + 1];
-            f[j][5] = gw[5 * B - 1];
-            f[j][6] = ge[6 * B - 1];
-            f[j][7] = ge[7 * B + 1];
-            f[j][8] = gw[8 * B + 1];
-        }
+        for (int j = K - 1; j >= 0; --j) tb_ring_pull<B>(rt, j + 1, o.pl[0], o.pl[1], o.pl[2], f[j]);
         if (r.strip_walls) {
 #pragma unroll
             for (int j = 0; j < K; ++j) {
@@ -726,9 +783,7 @@ LBM_HD void tb_fast_lane_fused(const TbArgs& a, const TbRow<T, B>& r, double* ri
             if (!act[j + 1]) continue;
             const int c = s - 2 * (j + 1);
             if (j + 2 < T) {
-                double* w = rt + (j + 1) * (TB_SLOTS * Q * B) + (c & (TB_SLOTS - 1)) * (Q * B);
-#pragma unroll
-                for (int i = 0; i < Q; ++i) w[i * B] = f[j][i];
+                tb_ring_put<B>(rt, j + 2, o.st[0], o.st[1], o.st[2], f[j]);
             } else {
                 if (a.m_rho) {  // (uniform; the last pass before an output only)
                     const long long g = (long long)c * a.L.ny + r.y;
@@ -743,13 +798,12 @@ LBM_HD void tb_fast_lane_fused(const TbArgs& a, const TbRow<T, B>& r, double* ri
         if (act[0]) {
             Moments m1;
             bad[0] |= tb_fast_cell<FORCED>(a, r.strip_walls, r.wall_b, r.wall_t, f1, m1);
-            double* w = rt + (s & (TB_SLOTS - 1)) * (Q * B);
-#pragma unroll
-            for (int i = 0; i < Q; ++i) w[i * B] = f1[i];
+            tb_ring_put<B>(rt, 1, o.st[0], o.st[1], o.st[2], f1);
         }
         pl = tb_opaque(pl + a.col_bytes);
         ps = tb_opaque(ps + a.col_bytes);
         if (pfp) pfp = tb_opaque(pfp + a.col_bytes);
+        tb_slots_advance<B>(o);
         TB_SYNC();
     }
 }
@@ -831,11 +885,8 @@ LBM_HD void tb_thread(const TbArgs& a, double* ring, int tid_, int strip_, int c
         // other steps keep writing the same values); the first step's barrier publishes it
         if (T > 1 && r.row_kind == 2) {
 #pragma unroll
-            for (int k = 1; k < T; ++k) {
-                if (!r.on[k - 1]) continue;
-                for (int slot = 0; slot < TB_SLOTS; ++slot)
-                    tb_ring_const<B>(ring + (k - 1) * (TB_SLOTS * Q * B) + slot * (Q * B) + r.tid, a, 2);
-            }
+            for (int k = 1; k < T; ++k)
+                if (r.on[k - 1]) tb_ring_fill<B>(ring + r.tid, k, a.bc.e);
         }
         // The fast lane takes every step whose columns are plain and unmasked: in a chunk that touches neither slab
         // edge that is the whole march (the stages switch themselves on and off at the chunk's ends), otherwise the
