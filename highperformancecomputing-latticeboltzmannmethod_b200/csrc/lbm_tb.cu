@@ -126,6 +126,9 @@ cudaError_t launch_one(TbArgs a, bool p2p, cudaStream_t s) {
             xc = 64;
             while (xc > 16 && (long long)strips * cdiv(ncols, xc) < 2LL * slots) xc /= 2;
         }
+        // a grid holds at most 65 535 blocks in y: wider chunks where a narrow LBM_B200_TB_XC asks for more
+        const int max_chunks = 65535 - (p2p ? 2 : 0);
+        if (cdiv(ncols, xc) > max_chunks) xc = cdiv(ncols, max_chunks);
         a.xc = xc;
         chunks = cdiv(ncols, xc);
     } else {

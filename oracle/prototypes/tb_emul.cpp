@@ -40,6 +40,7 @@ namespace {
 bool g_skew = true;  // which march (lbm_tb.cuh) the emulation runs; tb_set_skew
 int g_fast = 1;      // ... and whether the skewed march takes its fast lane
 bool g_fused = false;  // ... with the stages T..2 fused (k_tb<..., FUSED = true>)
+double g_force[2] = {0.0, 0.0};  // tb_set_force: a body force selects the FORCED = true thread program
 double* g_sink[3] = {nullptr, nullptr, nullptr};  // tb_set_macro_sink
 
 struct Slab {
@@ -99,7 +100,9 @@ void run_blocks(const TbArgs& a, int chunks) {
             for (int tid = 0; tid < B; ++tid)
                 th.emplace_back([&, tid] {
                     g_barrier = &bar;
-                    if (g_skew && g_fused) tb_thread<T, B, false, true, true>(a, ring.data(), tid, strip, chunk);
+                    // forced: the instantiation launch_forced (lbm_tb.cu) runs whatever the march settings
+                    if (g_force[0] != 0.0 || g_force[1] != 0.0) tb_thread<T, B, true>(a, ring.data(), tid, strip, chunk);
+                    else if (g_skew && g_fused) tb_thread<T, B, false, true, true>(a, ring.data(), tid, strip, chunk);
                     else if (g_skew) tb_thread<T, B, false, true>(a, ring.data(), tid, strip, chunk);
                     else tb_thread<T, B, false, false>(a, ring.data(), tid, strip, chunk);
                 });
@@ -107,16 +110,19 @@ void run_blocks(const TbArgs& a, int chunks) {
         }
 }
 
+template <int B>
+void run_pass_b(int depth, const TbArgs& a, int chunks) {
+    if (depth == 1) run_blocks<1, B>(a, chunks);
+    if (depth == 2) run_blocks<2, B>(a, chunks);
+    if (depth == 3) run_blocks<3, B>(a, chunks);
+}
+
+// B = 16 and 32 keep the emulated lattices small; 64 and 128 are block heights the device runs (128 the default).
 void run_pass(int depth, int B, const TbArgs& a, int chunks) {
-    if (B == 16) {
-        if (depth == 1) run_blocks<1, 16>(a, chunks);
-        if (depth == 2) run_blocks<2, 16>(a, chunks);
-        if (depth == 3) run_blocks<3, 16>(a, chunks);
-    } else {
-        if (depth == 1) run_blocks<1, 32>(a, chunks);
-        if (depth == 2) run_blocks<2, 32>(a, chunks);
-        if (depth == 3) run_blocks<3, 32>(a, chunks);
-    }
+    if (B == 16) run_pass_b<16>(depth, a, chunks);
+    else if (B == 64) run_pass_b<64>(depth, a, chunks);
+    else if (B == 128) run_pass_b<128>(depth, a, chunks);
+    else run_pass_b<32>(depth, a, chunks);
 }
 
 // One slab of the global state in the device Layout, both buffers, the mask with its deep flag (see tb_emulate for
@@ -184,6 +190,11 @@ extern "C" {
 // 0: the one-column-lag march; 1: the skewed march, every step on the general / lean step; 2: the skewed march with
 // its fast lane (what the device runs by default); 3: ... and the stages T..2 fused
 void tb_set_skew(int on) { g_skew = on != 0; g_fast = on >= 2; g_fused = on == 3; }
+// A body force (Fx, Fy) for the next tb_emulate calls: runs k_tb<T, B, FORCED = true> (0, 0: the plain program).
+void tb_set_force(double fx, double fy) {
+    g_force[0] = fx;
+    g_force[1] = fy;
+}
 // Where the LAST pass of the next tb_emulate call (world = 1) emits the moments its last stage's collisions read:
 // three arrays of nx*ny doubles in the slab's native order [x*ny + y] (TbArgs::m_rho / m_ux / m_uy); nullptr: off.
 void tb_set_macro_sink(double* rho, double* ux, double* uy) {
@@ -230,6 +241,8 @@ int tb_emulate(double* state, const unsigned char* solid, int nx, int ny, double
             a.dst = s.f[s.cur ^ 1].data();
             a.L = s.L;
             a.tau_inv = 1.0 / tau;
+            a.Fx = g_force[0];
+            a.Fy = g_force[1];
             a.first_bad = &first_bad;
             a.bad_iter = iter - 1;
             a.bc = bc0;

@@ -9,6 +9,7 @@ import pytest
 
 from oracle import oracle as O
 import parity_util as util
+import geometry_cases as G
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -18,6 +19,9 @@ CASES = {
     # odd ny: scalar bulk kernel, halo fused into the fix-up kernel instead of the bulk launch
     "periodic": O.Case(nx=96, ny=40, cylinder_x=0.02, cylinder_radius=0.2, output_frequency=6, inlet_velocity=0.04),  # flags=1 in the worker
     "odd": O.Case(nx=128, ny=47, cylinder_x=0.5, cylinder_radius=0.2, output_frequency=6, inlet_velocity=0.04),
+    # several strips: the disc is centred on the face x = 64 (and lies across x = 32 .. 96 of a 4-slab run), and its
+    # last row is the first row of the block of strip 1 at depths 2 / 3, B = 128 (tests/geometry_cases.py)
+    "strip_edge": G.disc(128, 300, 64, G.block_lo(128, 3, 1) - 20, 20, output_frequency=6, inlet_velocity=0.04),
 }
 
 

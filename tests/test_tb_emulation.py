@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
+import geometry_cases as G
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "oracle", "prototypes", "libtbemul.so")
@@ -31,6 +32,7 @@ def emu(request):
     """The marches of lbm_tb.cuh: the skewed one (stage k two columns behind stage k-1, the default) with and without
     its fast lane for plain stretches (and with the later stages of the fast lane fused), and the one-column-lag one with its second cell of prefetched registers."""
     L = C.CDLL(LIB)
+    L.tb_set_force.argtypes = [C.c_double, C.c_double]
     L.tb_set_skew({"skewed": 2, "skewed_fused": 3, "skewed_no_fast_lane": 1, "one_column_lag": 0}[request.param])
     L.tb_emulate.restype = C.c_int
     L.tb_emulate.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int,
@@ -198,3 +200,77 @@ def test_the_last_pass_emits_the_moments_of_its_last_collision(emu, depths):
     for mine, want in zip(sink, (o.rho, o.ux, o.uy)):
         mine = mine.reshape(case.nx, case.ny).T  # native [x*ny + y] -> [y, x]
         assert np.array_equal(mine[:, 1:-1], np.asarray(want)[:, 1:-1])
+
+
+def _strip_edge_params():
+    """The obstacle-row cases of tests/geometry_cases.py at the shipped block height, B = 128 (strip 1's block edges),
+    with the passes of the depths they were derived for."""
+    out = []
+    for depth, depths in ((1, (1, 1)), (3, (3, 2))):
+        for name in G.row_edge_cases(G.DEFAULT_B, depth):
+            out.append(pytest.param(depth, name, depths, id=name))
+    return out
+
+
+@pytest.mark.parametrize("depth,name,depths", _strip_edge_params())
+def test_strip_edges_at_the_shipped_block_height(emu, depth, name, depths):
+    """B = 128 (and xc = 8, so that every block of 128 threads has a short march): the obstacle's rows just inside and
+    just outside the block of strip 1, which decides whether that block looks at the mask at all."""
+    case = G.row_edge_cases(G.DEFAULT_B, depth)[name]
+    assert case.nx <= 40
+    o = O.Oracle(case)
+    o.f_current[...] = random_f_current(case, 6)
+    o.run(1)
+    src, solid = o.f_next.copy(), padded_solid(o, case)
+    got, bad = emulate(emu, case, src, solid, depths, B=G.DEFAULT_B, xc=8)
+    o.run(sum(depths))
+    assert bad == 0x7fffffff
+    diff = (got[1:-1, 1:-1] != o.f_next[1:-1, 1:-1]).any(axis=2)
+    where = np.argwhere(diff)
+    assert not diff.any(), "%d cells differ, first (y, x) = %s, strip %d" % (
+        len(where), tuple(where[0]), where[0][0] // G.rows_per_strip(G.DEFAULT_B, depth))
+
+
+@pytest.mark.parametrize("B", [64, 128])
+def test_the_default_case_at_block_heights_the_device_runs(B):
+    """Multi-strip at B = 64 (ny = 150: three strips) and B = 128, the skewed march with its fast lane."""
+    L = C.CDLL(LIB)
+    L.tb_emulate.restype = C.c_int
+    L.tb_emulate.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int,
+                             C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+    L.tb_set_skew(2)
+    case = G.disc(36, 150 if B == 64 else 260, 12, G.rows_per_strip(B, 3), 9, output_frequency=5)
+    o = O.Oracle(case)
+    o.f_current[...] = random_f_current(case, 8)
+    o.run(1)
+    src, solid = o.f_next.copy(), padded_solid(o, case)
+    got, bad = emulate(L, case, src, solid, (3, 1, 2), B=B, xc=6)
+    o.run(6)
+    assert bad == 0x7fffffff
+    assert np.array_equal(got[1:-1, 1:-1], o.f_next[1:-1, 1:-1])
+
+
+@pytest.mark.parametrize("flags", [0, 1, 2, 3])
+@pytest.mark.parametrize("B,name", [(16, "64x32"), (32, "70x33")])
+def test_forced_passes_are_self_consistent(emu, flags, B, name):
+    """A body force (Fx and Fy) selects k_tb<T, B, FORCED = true>, which has no reference: depth-2 / depth-3 passes
+    against single depth-1 passes of the same code, with the obstacle, walls, inlet and outlet (flags 0) and the
+    periodic edges, over several strips and chunks."""
+    case = CASES[name]
+    o = O.Oracle(case)
+    rng = np.random.default_rng(2)
+    w = np.array([4 / 9] + [1 / 9] * 4 + [1 / 36] * 4)
+    state = np.ascontiguousarray(w * (1.0 + 0.05 * rng.standard_normal((case.ny + 2, case.nx + 2, 9))))
+    solid = padded_solid(o, case)
+    state[solid != 0] = w
+    emu.tb_set_force.argtypes = [C.c_double, C.c_double]
+    plain, _ = emulate(emu, case, state, solid, (1,) * 6, flags=flags, B=B, xc=1000)
+    emu.tb_set_force(2e-5, -3e-5)
+    try:
+        ref, _ = emulate(emu, case, state, solid, (1,) * 6, flags=flags, B=B, xc=1000)
+        assert not np.array_equal(ref[1:-1, 1:-1], plain[1:-1, 1:-1])  # the force does act
+        for depths in ((2, 2, 2), (3, 3), (2, 1, 3)):
+            got, _ = emulate(emu, case, state, solid, depths, flags=flags, B=B, xc=7)
+            assert np.array_equal(got[1:-1, 1:-1], ref[1:-1, 1:-1]), depths
+    finally:
+        emu.tb_set_force(0.0, 0.0)
