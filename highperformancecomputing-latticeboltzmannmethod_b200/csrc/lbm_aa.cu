@@ -420,7 +420,7 @@ __device__ __forceinline__ void aa_macros_cell(const AaObserve& o, int x, int y,
     if (o.fresh) {
         rho = 1.0;
         uy = 0.0;
-        ux = solid ? 0.0 : (o.shear_wave ? o.u0 * sin(2.0 * 3.14159265358979323846 * (double)y / (double)L.ny) : o.bc.u_in);
+        ux = solid ? 0.0 : (o.shear_wave ? o.u0 * sin(2.0 * 3.14159265358979323846 * (double)y / (double)L.ny) : o.u0);  // Grid::initialise(inlet_u)
         return;
     }
     if (solid) {

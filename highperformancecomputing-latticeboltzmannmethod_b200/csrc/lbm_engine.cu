@@ -121,6 +121,11 @@ struct lbm_solver {
     double* d_ring_out = nullptr;
 
     BcArgs bc{};
+    // The parameters the last iteration ran with.  lbm_set_params replaces h->p and h->bc at once, but the boundary
+    // rules of the last iteration are applied by the NEXT launch (it pulls that iteration's populations), and the
+    // observers rebuild that iteration's state: both use these (mark_run copies them when an iteration is launched).
+    double run_tau_inv = 0.0, run_Fx = 0.0, run_Fy = 0.0;
+    BcArgs run_bc{};
     double init_u = 0.0;
     int variant = BULK_TB;
     bool overlap = true;
@@ -194,13 +199,21 @@ StepArgs step_args(lbm_handle h, const double* src, double* dst, int bad_iter, i
     return a;
 }
 
+// Every launch of an iteration ends with this: from now on its parameters are the ones still owed (see run_bc).
+void mark_run(lbm_handle h) {
+    h->run_tau_inv = 1.0 / h->p.tau;
+    h->run_Fx = h->p.body_force_x;
+    h->run_Fy = h->p.body_force_y;
+    h->run_bc = h->bc;
+}
+
 ObserveArgs observe_args(lbm_handle h) {
     ObserveArgs o;
     o.cur = h->f[h->cur];
     o.prev = h->f[h->cur ^ 1];
     o.L = h->L;
     o.mask = h->d_mask;
-    o.bc = h->bc;
+    o.bc = h->run_bc;
     o.cur_is_next = h->cur_is_next;
     o.prev_is_next = h->prev_is_next;
     o.fresh = h->fresh;
@@ -235,7 +248,7 @@ AaObserve aa_observe(lbm_handle h) {
     o.f = h->f[0];
     o.L = h->L;
     o.mask = h->d_mask;
-    o.bc = h->bc;
+    o.bc = h->run_bc;
     o.phase = h->aa_phase;
     o.cur_is_next = h->cur_is_next;
     o.fresh = h->fresh;
@@ -248,9 +261,9 @@ AaObserve aa_observe(lbm_handle h) {
     o.east_zero = (h->periodic_x || h->east >= 0) ? 0 : 1;
     o.shear_wave = (h->p.flags & LBM_FLAG_SHEAR_WAVE_INIT) ? 1 : 0;
     o.u0 = h->init_u;
-    o.tau_inv = 1.0 / h->p.tau;
-    o.Fx = h->p.body_force_x;
-    o.Fy = h->p.body_force_y;
+    o.tau_inv = h->run_tau_inv;
+    o.Fx = h->run_Fx;
+    o.Fy = h->run_Fy;
     return o;
 }
 
@@ -660,7 +673,7 @@ int step_one_aa(lbm_handle h) {
     const bool wrap_x1 = h->periodic_x && h->world == 1;  // the wrap stays inside this GPU
     const int open_x = ((h->periodic_x || h->west >= 0) ? 1 : 0) | ((h->periodic_x || h->east >= 0) ? 2 : 0);
     if (!odd) {
-        CU(h, launch_aa_fix_even(a, h->bc, h->d_ring, h->n_ring, h->d_solids, solids_to_reset(h, !a.first, true), h->stream));
+        CU(h, launch_aa_fix_even(a, h->run_bc, h->d_ring, h->n_ring, h->d_solids, solids_to_reset(h, !a.first, true), h->stream));
         h->launches += 2;
         if (wrap_x1) { CU(h, launch_wrap(h->f[0], L, 1, 0, h->stream)); h->launches += 1; }
         if (multi) {
@@ -678,7 +691,7 @@ int step_one_aa(lbm_handle h) {
         // Constant fill last: across an open edge the reverse wrap / halo also carries what solid cells
         // pushed, and the fill must overwrite that.
         const bool wrap = wrap_x1 || h->periodic_y || multi;
-        CU(h, launch_aa_fix_odd(a, h->bc, h->d_ring, h->n_ring, h->d_fills, wrap ? 0 : h->n_fill, h->d_ring_out, open_x,
+        CU(h, launch_aa_fix_odd(a, h->run_bc, h->d_ring, h->n_ring, h->d_fills, wrap ? 0 : h->n_fill, h->d_ring_out, open_x,
                                 h->periodic_y ? 1 : 0, h->stream));
         h->launches += 2;
         if (wrap) {
@@ -695,10 +708,11 @@ int step_one_aa(lbm_handle h) {
                 int rc = join_halo(h);
                 if (rc) return rc;
             }
-            CU(h, launch_aa_fix_odd(a, h->bc, h->d_ring, 0, h->d_fills, h->n_fill, h->d_ring_out, 0, 0, h->stream));
+            CU(h, launch_aa_fix_odd(a, h->run_bc, h->d_ring, 0, h->d_fills, h->n_fill, h->d_ring_out, 0, 0, h->stream));
             h->launches += (h->n_fill ? 1 : 0);
         }
     }
+    mark_run(h);
     h->aa_phase ^= 1;
     h->prev_is_next = h->cur_is_next;
     h->cur_is_next = true;
@@ -735,7 +749,7 @@ TbArgs tb_args(lbm_handle h, const double* src, double* dst, int bad_iter, int w
     a.Fy = h->p.body_force_y;
     a.first_bad = h->d_first_bad;
     a.bad_iter = bad_iter;
-    a.bc = h->bc;
+    a.bc = h->run_bc;  // the rules of the iteration the first stage pulls
     a.mask = h->d_mask;
     a.mask_lo = h->mask_lo;
     a.mask_hi = h->mask_hi;
@@ -861,6 +875,7 @@ int step_tb(lbm_handle h, int depth, bool emit) {
         h->launches += 1;
         h->pending.push_back({last, slot});
     }
+    mark_run(h);
     h->cur ^= 1;
     h->prev_is_next = depth > 1 ? true : h->cur_is_next;
     h->cur_is_next = true;
@@ -883,6 +898,9 @@ int plan_depth(int iter, int remaining, int of, int max_depth, bool cur_is_next)
 }
 
 int next_depth(lbm_handle h, int remaining) {
+    // A pass applies one set of boundary rules: after lbm_set_params changed u_in, the iteration that still owes the
+    // old inlet rule is a pass of its own.
+    if (h->run_bc.u_in != h->bc.u_in) return 1;
     return plan_depth(h->iter, remaining, h->p.output_frequency, h->tb_depth, h->cur_is_next);
 }
 
@@ -925,7 +943,7 @@ int step_one(lbm_handle h) {
         const bool fused = bulk_p2p_supported(h->variant, a);
         if (!fused) {
             CU(h, bulk(0, L.lnx));
-            CU(h, launch_fixup_p2p(pull, a, h->bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
+            CU(h, launch_fixup_p2p(pull, a, h->run_bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
                                    h->d_solids, solids_to_reset(h, pull, false), h->d_mask,
                                    px, h->stream));
         } else {
@@ -934,7 +952,7 @@ int step_one(lbm_handle h) {
                 cudaEventCreate(&e0);
                 cudaEventCreate(&e1);
                 cudaEventRecord(e0, h->stream);
-                CU(h, launch_bulk_p2p(pull, a, h->bc, h->d_mask, px, h->stream));
+                CU(h, launch_bulk_p2p(pull, a, h->run_bc, h->d_mask, px, h->stream));
                 cudaEventRecord(e1, h->stream);
                 h->bulk_events.push_back(e0);
                 h->bulk_events.push_back(e1);
@@ -942,9 +960,9 @@ int step_one(lbm_handle h) {
                 h->bulk_timed_cells += (long long)L.lnx * L.ny - h->n_deep;
                 h->bulk_timed_updates += (long long)L.lnx * L.ny - h->n_deep;
             } else {
-                CU(h, launch_bulk_p2p(pull, a, h->bc, h->d_mask, px, h->stream));
+                CU(h, launch_bulk_p2p(pull, a, h->run_bc, h->d_mask, px, h->stream));
             }
-            CU(h, launch_fixup(pull, a, h->bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
+            CU(h, launch_fixup(pull, a, h->run_bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
                                h->d_solids, solids_to_reset(h, pull, false), h->stream));
         }
         h->launches += 2;
@@ -956,10 +974,10 @@ int step_one(lbm_handle h) {
         // Only the edge kernel reads ghost columns; it comes last, a whole interior kernel after the
         // exchange it depends on was issued, so its wait is satisfied long before it is reached.
         CU(h, bulk(1, L.lnx - 1));
-        CU(h, launch_fixup(pull, a, h->bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
+        CU(h, launch_fixup(pull, a, h->run_bc, h->d_ring + h->n_ring_edge, h->n_ring - h->n_ring_edge,
                            h->d_solids, solids_to_reset(h, pull, false), h->stream));
         CU(h, cudaStreamWaitEvent(h->stream, h->ev_comm, 0));
-        CU(h, launch_edge(pull, a, h->bc, h->d_mask, h->stream));
+        CU(h, launch_edge(pull, a, h->run_bc, h->d_mask, h->stream));
         CU(h, cudaEventRecord(h->ev_edge, h->stream));
         CU(h, cudaStreamWaitEvent(h->comm_stream, h->ev_edge, 0));
         int rc = exchange(h, dst, h->comm_stream);
@@ -968,7 +986,7 @@ int step_one(lbm_handle h) {
         h->launches += 3;
     } else {
         CU(h, bulk(0, L.lnx));
-        CU(h, launch_fixup(pull, a, h->bc, h->d_ring, h->n_ring, h->d_solids, solids_to_reset(h, pull, false), h->stream));
+        CU(h, launch_fixup(pull, a, h->run_bc, h->d_ring, h->n_ring, h->d_solids, solids_to_reset(h, pull, false), h->stream));
         h->launches += 2;
         if (multi) {
             int rc = exchange(h, dst, h->stream);
@@ -1013,6 +1031,7 @@ int step_one(lbm_handle h) {
         h->launches += 1;
         h->custom_pending -= 1;
     }
+    mark_run(h);
     h->cur ^= 1;
     h->prev_is_next = h->cur_is_next;
     h->cur_is_next = true;
@@ -1046,6 +1065,9 @@ int ensure_macros(lbm_handle h) {
         int rc = ensure_native_macros(h);
         if (rc) return rc;
         TbArgs a = tb_args(h, h->f[h->cur ^ 1], h->f[h->cur], h->iter - h->lag - 1, 0);
+        a.tau_inv = h->run_tau_inv;  // (the pass ran with these even if lbm_set_params has replaced them since)
+        a.Fx = h->run_Fx;
+        a.Fy = h->run_Fy;
         a.first_bad = h->d_first_bad_all;  // (already judged by the pass itself; keep the verdict word untouched)
         a.m_rho = h->d_mrho;
         a.m_ux = h->d_mux;
@@ -1100,13 +1122,20 @@ int check_pending(lbm_handle h) {
     { int rc_ = join_halo(h); if (rc_) return rc_; }
     if (h->variant == BULK_TB && !h->custom_state) {
         TbArgs t = tb_args(h, h->f[h->cur], h->f[h->cur ^ 1], h->iter - 1, 0);
+        t.tau_inv = h->run_tau_inv;
+        t.Fx = h->run_Fx;
+        t.Fy = h->run_Fy;
         CU(h, launch_tb(1, t, false, h->stream));
         h->launches += 1;
         return LBM_OK;
     }
     StepArgs a = step_args(h, h->f[h->cur], h->f[h->cur ^ 1], h->iter - 1, 0);
+    a.tau_inv = h->run_tau_inv;
+    a.Fx = h->run_Fx;
+    a.Fy = h->run_Fy;
+    a.forced = (a.Fx != 0.0 || a.Fy != 0.0) ? 1 : 0;
     CU(h, launch_bulk(BULK_VEC2, true, a, h->stream, 0, h->L.lnx));
-    CU(h, launch_fixup(true, a, h->bc, h->d_ring, h->n_ring, nullptr, 0, h->stream));
+    CU(h, launch_fixup(true, a, h->run_bc, h->d_ring, h->n_ring, nullptr, 0, h->stream));
     h->launches += 2;
     return LBM_OK;
 }
@@ -1372,6 +1401,9 @@ int lbm_setup_geometry(lbm_handle h, int* solid_count) {
     int rc = build_geometry(h);
     if (rc) return rc;
     if (solid_count) *solid_count = h->n_solid;
+    // The buffers still hold the old geometry's state (a cell that became solid holds a different value in each):
+    // the next step needs lbm_initialise or lbm_upload_f first.
+    h->initialised = false;
     return LBM_OK;
 }
 
@@ -1414,6 +1446,7 @@ int lbm_initialise(lbm_handle h, double inlet_u) {
     h->macros_native_iter = -1;
     h->custom_state = false;
     h->custom_pending = 0;
+    mark_run(h);
     h->pending.clear();
     h->force_log.clear();
     if (h->p2p) return slab_barrier(h);  // every slab initialised before any neighbour pushes a halo into it
@@ -1668,6 +1701,10 @@ int lbm_upload_f(lbm_handle h, const double* aos, int iteration) {
     h->macros_valid = false;
     h->lag = 1;
     h->macros_native_iter = -1;
+    // The ghost rows were just reset in both buffers, and the first step resets every solid cell: values the caller
+    // wrote into f_next (lbm_upload_f_next) go into the destinations of the next two steps again.
+    if (h->custom_state && h->n_custom) h->custom_pending = 2;
+    mark_run(h);
     if (h->p2p) return slab_barrier(h);
     return LBM_OK;
 }

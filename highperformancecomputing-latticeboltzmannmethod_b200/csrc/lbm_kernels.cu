@@ -441,7 +441,7 @@ __device__ __forceinline__ void macros_cell(const ObserveArgs& o, int x, int y, 
         else if (o.shear_wave)
             ux = o.u0 * sin(2.0 * 3.14159265358979323846 * (double)y / (double)L.ny);
         else
-            ux = o.bc.u_in;
+            ux = o.u0;  // the velocity Grid::initialise(inlet_u) was given, not the params' inlet velocity
         return;
     }
     if (solid) {  // rho stays 1.0 from the constructor; include/LBMSolver.h:260-261

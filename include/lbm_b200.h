@@ -108,12 +108,22 @@ int lbm_get_info(lbm_handle h, lbm_info* out);
 int lbm_bootstrap_env(int* rank, int* world, int* local_rank, void* nccl_unique_id_out128);
 /* Change tau / inlet velocity / cylinder / output_frequency / body force after creation (the
  * reference's Grid is constructed from nx, ny alone and learns the rest in setup_geometry and
- * initialise, include/LBMGrid.h:57,152,185).  nx, ny and periodicity cannot change. */
+ * initialise, include/LBMGrid.h:57,152,185).  nx, ny and periodicity cannot change.
+ * On a running handle the new values apply from the next iteration on, as if they had been changed between two
+ * iterations of the reference: the observers still show the state the last iteration left, computed with the
+ * parameters it ran with (its inlet rule, tau and body force), and the next iteration applies the old inlet rule to
+ * the populations it pulls (the reference's boundary pass of the last iteration).  A new obstacle takes effect with
+ * lbm_setup_geometry. */
 int lbm_set_params(lbm_handle h, const lbm_params* p);
 
 /* ---- set-up: Solver::initialise (include/LBMSolver.h:31-41) ---- */
-int lbm_setup_geometry(lbm_handle h, int* solid_count); /* Grid::setup_geometry, LBMGrid.h:152-183 */
-int lbm_initialise(lbm_handle h, double inlet_u);       /* Grid::initialise,     LBMGrid.h:185-246 */
+/* Grid::setup_geometry, LBMGrid.h:152-183.  Rebuilds the mask and every table derived from it.  The populations are
+ * those of the old geometry, so the handle is left uninitialised: lbm_step / lbm_run fail with LBM_ERR_INVALID until
+ * lbm_initialise (or lbm_upload_f) gives it a state. */
+int lbm_setup_geometry(lbm_handle h, int* solid_count);
+/* Grid::initialise, LBMGrid.h:185-246: populations eq(1, inlet_u, 0), fluid ux = inlet_u, iteration 0, no stability
+ * verdict, no forces rows, caller-written f_next values dropped.  The inlet rule keeps the params' inlet_velocity. */
+int lbm_initialise(lbm_handle h, double inlet_u);
 
 /* ---- the hot path: the loop body of Solver::run (include/LBMSolver.h:48-76) ---- */
 /* Advance n reference iterations asynchronously: fused pull+boundary+collide kernels, the halo
@@ -171,7 +181,12 @@ int lbm_download_macros(lbm_handle h, double* rho, double* ux, double* uy);
 int lbm_download_solid(lbm_handle h, unsigned char* mask);
 /* Replace the state by a given f_current (padded AoS; ghost entries ignored).  Used for
  * restart and for parity tests on seeded random states.  `iteration` is the reference timestep
- * the next lbm_step will execute. */
+ * the next lbm_step will execute.  Allowed at any point of a run, with any kernel variant and pass depth: the run
+ * goes on as the reference's would after writing f_current at that iteration boundary.  f_next keeps what the
+ * reference's f_next holds there: w in solid cells and the initial equilibrium in the S/N ghost rows, or the values
+ * an earlier lbm_upload_f_next wrote.  Until the next iteration the observers derived from f_next describe the
+ * uploaded state as right after Grid::initialise: lbm_download_f(LBM_F_NEXT) returns f_current, lbm_get_forces sums
+ * its links, rho / u are its moments (1 / 0 / 0 in solid cells), and lbm_check_stability reports no failure. */
 int lbm_upload_f(lbm_handle h, const double* f_current_aos_padded, int iteration);
 
 /* Grid::f_next written by the caller (LBMGrid.h:119-121 hands out a mutable reference).  At an iteration boundary of
@@ -179,8 +194,9 @@ int lbm_upload_f(lbm_handle h, const double* f_current_aos_padded, int iteration
  * only the values of SOLID cells and of the S/N GHOST ROWS (corners included) live on: the next iteration's streaming
  * and every later one pull them.  Exactly those values are taken from the image (fluid cells and the W/E ghost
  * columns, which the exchange rewrites every step, are ignored) and take effect with the next iteration, as in the
- * reference; lbm_download_f shows them after that iteration.  From this call on the handle runs the one-iteration
- * kernels: the temporally blocked passes build the default constants in.  Single-rank semantics per slab. */
+ * reference; lbm_download_f shows them after that iteration.  They stay through later lbm_upload_f calls, until
+ * lbm_initialise.  From this call on the handle runs the one-iteration kernels: the temporally blocked passes build
+ * the default constants in.  Single-rank semantics per slab. */
 int lbm_upload_f_next(lbm_handle h, const double* f_next_aos_padded);
 
 /* ---- async output: replaces the MPI gathers of Solver::write_vtk_frame (LBMSolver.h:269-362)
